@@ -10,9 +10,8 @@ as the reported CPU baseline -- never as the measured GPU path.
 
 Pinning status: the reference ships no tests and no golden vectors (SURVEY.md
 section 8c), so the oracle is pinned against outputs of the reference ITSELF,
-imported in the build container from /root/reference by
+imported through ``oracle/reference_import.py`` by
 ``oracle/make_golden.py`` (committed), which writes ``tests/golden/*.npz``.
 ``tests/test_oracle_vs_golden.py`` checks the restatement against those
-fixtures on every run; ``tests/test_oracle_vs_reference.py`` checks it against
-the live reference when /root/reference is present.
+fixtures on every run.
 """

@@ -1,6 +1,6 @@
 """Generate tests/golden/*.npz by running the UNMODIFIED reference on CPU
-(TEST INFRASTRUCTURE; run in the build container only:
-``python -m oracle.make_golden``).
+(TEST INFRASTRUCTURE; ``LANEFIT_REFERENCE=<checkout of the original project> python -m oracle.make_golden``;
+without the variable, oracle/reference_import.py picks the oracle/_ref/ install or the default checkout).
 
 The reference has no golden vectors of its own (SURVEY.md 8c), so these files
 are the pin: outputs of the reference's own modules (float32 = its arithmetic,
