@@ -27,44 +27,56 @@ def build_net(L, order, mask_pct, B):
     return Net(args), args
 
 
-def run_full_path(name, tol=1e-4, enforce=True, golden_dir=GOLDEN):
-    """Run case `name` (net_l2_d2 / net_l4_d3) in the CURRENT ops_net.CONV_MODE.  Returns a report dict with the worst
-    norm-wise errors (ours vs fp64, reference-fp32 vs fp64); with `enforce` every gate is asserted."""
-    from lanedetection_end2end_b200.Loss_crit import backprojection_loss
-    g = np.load(os.path.join(golden_dir, name + ".npz"))
-    meta = json.loads(str(g["meta"]))
-    L, order, B = meta["L"], meta["order"], meta["B"]
-    model, args = build_net(L, order, meta["mask_pct"], B)
-    sd = model.state_dict()
-    for k, v in inputs.make_erfnet_params(3, L, seed=meta["param_seed"]).items():
-        sd[k] = torch.from_numpy(v)
-    model.load_state_dict(sd)
-    model = model.cuda().train()
-    for m in model.modules():
-        if hasattr(m, "dropout"):
-            m.dropout.p = 0
-    # the grid must be bit-identical to the reference's (same torch ops on the same cv2 homography)
-    np.testing.assert_array_equal(model.grid[0].cpu().numpy(), np.load(os.path.join(golden_dir, "lsq_bp_l2_d2.npz"))["grid0"])
-    x = torch.from_numpy(inputs.make_images(B, 256, 512, seed=meta["image_seed"])).cuda()
-    xgt_np, valid_np = inputs.make_loss_targets(B, 4, seed=meta["target_seed"])
-    xgt, valid = torch.from_numpy(xgt_np).cuda(), torch.from_numpy(valid_np).cuda()
-    taps, hooks = {}, []
-    mods = {"encoder.initial_block": model.net.encoder.initial_block, "decoder.output_conv": model.net.decoder.output_conv}
-    mods.update({"encoder.layers.%d" % i: l for i, l in enumerate(model.net.encoder.layers)})
-    mods.update({"decoder.layers.%d" % i: l for i, l in enumerate(model.net.decoder.layers)})
-    for n, mod in mods.items():
-        hooks.append(mod.register_forward_hook(lambda _m, _i, o, n=n: taps.__setitem__(n, o)))
-    out = model(x, torch.zeros(B, 4), True)
-    for h in hooks:
-        h.remove()
-    betas = [b for b in out[:4] if b is not None]
-    assert len(betas) == L and betas[0].dtype == torch.float64 and betas[0].shape == (B, order + 1, 1)
-    crit = backprojection_loss(args)
-    loss = sum(crit(betas[l], xgt[:, l], valid[:, l])[0] for l in range(L)) / L
-    loss.backward()
-    torch.cuda.synchronize()
+class FullPathCase:
+    """Case `name` of the whole-path goldens, ready to run: the fixture `g` and its `meta`, the model with the golden
+    parameters (cuda:0, train mode, dropout p = 0), the reference's `args`, and the inputs x, xgt, valid on cuda:0."""
 
-    rep = {"case": name, "act": (0.0, 0.0, ""), "grad": (0.0, 0.0, ""), "grad_significant": (0.0, 0.0, "")}
+    def __init__(self, name, golden_dir=GOLDEN):
+        g = np.load(os.path.join(golden_dir, name + ".npz"))
+        meta = json.loads(str(g["meta"]))
+        L, order, B = meta["L"], meta["order"], meta["B"]
+        model, args = build_net(L, order, meta["mask_pct"], B)
+        sd = model.state_dict()
+        for k, v in inputs.make_erfnet_params(3, L, seed=meta["param_seed"]).items():
+            sd[k] = torch.from_numpy(v)
+        model.load_state_dict(sd)
+        model = model.cuda().train()
+        for m in model.modules():
+            if hasattr(m, "dropout"):
+                m.dropout.p = 0
+        # the grid must be bit-identical to the reference's (same torch ops on the same cv2 homography)
+        np.testing.assert_array_equal(model.grid[0].cpu().numpy(), np.load(os.path.join(golden_dir, "lsq_bp_l2_d2.npz"))["grid0"])
+        self.name, self.g, self.meta, self.model, self.args = name, g, meta, model, args
+        self.L, self.order, self.B = L, order, B
+        self.x = torch.from_numpy(inputs.make_images(B, 256, 512, seed=meta["image_seed"])).cuda()
+        xgt_np, valid_np = inputs.make_loss_targets(B, 4, seed=meta["target_seed"])
+        self.xgt, self.valid = torch.from_numpy(xgt_np).cuda(), torch.from_numpy(valid_np).cuda()
+
+    def tap_modules(self):
+        """The modules whose outputs the fixture samples, by fixture name."""
+        net = self.model.net
+        mods = {"encoder.initial_block": net.encoder.initial_block, "decoder.output_conv": net.decoder.output_conv}
+        mods.update({"encoder.layers.%d" % i: l for i, l in enumerate(net.encoder.layers)})
+        mods.update({"decoder.layers.%d" % i: l for i, l in enumerate(net.decoder.layers)})
+        return mods
+
+    def hook_taps(self):
+        """Forward hooks that store each tapped module's latest output in the returned dict; returns (taps, handles)."""
+        taps, hooks = {}, []
+        for n, mod in self.tap_modules().items():
+            hooks.append(mod.register_forward_hook(lambda _m, _i, o, n=n: taps.__setitem__(n, o)))
+        return taps, hooks
+
+
+def compare_full_path(case, taps, betas, loss, tol=1e-4, enforce=True):
+    """Compare one training step of `case.model` with the golden: the sampled activations in `taps`, the curve
+    coefficients `betas` (L tensors [B, order+1, 1] float64), the `loss`, every parameter gradient and the BatchNorm
+    running statistics after one step.  Returns a report dict with the worst norm-wise errors (ours vs fp64,
+    reference-fp32 vs fp64); with `enforce` every gate is asserted."""
+    g, model = case.g, case.model
+    assert len(betas) == case.L and betas[0].dtype == torch.float64 and betas[0].shape == (case.B, case.order + 1, 1)
+
+    rep = {"case": case.name, "act": (0.0, 0.0, ""), "grad": (0.0, 0.0, ""), "grad_significant": (0.0, 0.0, "")}
 
     def check(ok, msg):
         if enforce:
@@ -114,3 +126,21 @@ def run_full_path(name, tol=1e-4, enforce=True, golden_dir=GOLDEN):
             ref = g["buf_f64/" + n]
             check(np.abs(b.cpu().numpy() - ref).max() <= 1e-4 * max(np.abs(ref).max(), 1e-3), n)
     return rep
+
+
+def run_full_path(name, tol=1e-4, enforce=True, golden_dir=GOLDEN):
+    """Run case `name` (net_l2_d2 / net_l4_d3 / net_l2_d2_b32) eagerly in the CURRENT ops_net.CONV_MODE: one forward
+    and backward through the calls the reference's main.py makes, then compare_full_path."""
+    from lanedetection_end2end_b200.Loss_crit import backprojection_loss
+    case = FullPathCase(name, golden_dir)
+    model, B, L = case.model, case.B, case.L
+    taps, hooks = case.hook_taps()
+    out = model(case.x, torch.zeros(B, 4), True)
+    for h in hooks:
+        h.remove()
+    betas = [b for b in out[:4] if b is not None]
+    crit = backprojection_loss(case.args)
+    loss = sum(crit(betas[l], case.xgt[:, l], case.valid[:, l])[0] for l in range(L)) / L
+    loss.backward()
+    torch.cuda.synchronize()
+    return compare_full_path(case, taps, betas, loss, tol, enforce)
